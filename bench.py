@@ -2,7 +2,7 @@
 """bench.py -- flow-rows/s classified per model on B200 (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload gnb|logistic|kmeans|forest|forest_hbm|knn|svc]
-                    [--impl reference] [--no-extras]
+                    [--impl reference] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -12,6 +12,9 @@ A "step" is one pass of the hot path over one batch.  Batches rotate through a r
 float32 and already resident in HBM for `value`; `e2e` goes through the public estimator call with pinned HOST
 buffers (H2D rows + D2H labels inside the timed region).  The other models/configs are measured in the same run
 and reported under "models" (each with its own roofline and e2e), so the single line carries every model.
+`--steps K` is the number of timed steps of every model's device-resident measurement.  `--dump-outputs DIR` writes
+the labels of each model's last timed step; inputs and models are seeded, so two builds run with the same arguments
+can be compared output for output.
 `cpu_baseline` / `--impl reference` time scikit-learn -- the library whose predict() the reference calls at
 traffic_classifier.py:106 -- on the box's host cores.
 """
@@ -29,6 +32,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the bench leaves the tree as it found it (it may be read-only)
 
 L2_BYTES = 126 << 20
 # the arithmetic each kernel computes in (a description, not a precision claim: labels are the fp64 definition's everywhere)
@@ -37,6 +41,8 @@ DTYPES = {"gnb": "f32 certified pre-pass + f64 re-evaluation of uncertified rows
           "svc": "bf16x3 tensor-core distances + f32 exp/sums with a certificate + f64 re-evaluation of uncertified rows"}
 OPTIONS = []   # (key, value) pairs for tcsdn_set_option on every estimator the bench creates (--set-option)
 WORKLOADS = ("gnb", "gnb_100m", "logistic", "kmeans", "forest", "forest_hbm", "forest_hbm2", "knn", "svc")
+# --dump-outputs keeps at most this many rows' labels per workload: 4 MiB of float32 each, nine workloads stay under 64 MiB
+DUMP_ROWS = 1 << 20
 
 
 # ----------------------------------------------------------------------------- workload definitions
@@ -389,8 +395,17 @@ def measure_with_gather(w, steps, world, device):
     return dict(best, nccl_allgather=nccl, fused_peer_memory=fused)
 
 
-def measure_gpu(w, steps, warmup, world, device, peaks, extras_light=False, clock_probe_s=0.0):
-    """Device-resident timing (`value`) + end-to-end timing (`e2e`) of one workload on this rank."""
+def dump_sample(rows):
+    """Row indices --dump-outputs keeps of a `rows`-row step: None (all of them) up to DUMP_ROWS, else a fixed, seeded,
+    sorted sample of DUMP_ROWS rows (the same rows on every run with the same arguments)."""
+    if rows <= DUMP_ROWS:
+        return None
+    return np.sort(np.random.default_rng(0).choice(rows, DUMP_ROWS, replace=False))
+
+
+def measure_gpu(w, steps, warmup, world, device, peaks, extras_light=False, clock_probe_s=0.0, keep_labels=False):
+    """Device-resident timing (`value`) + end-to-end timing (`e2e`) of one workload on this rank.  keep_labels: also
+    return the label indices of the last timed step (the rows dump_sample picks) as float32, for --dump-outputs."""
     import torch
     from traffic_classifier_sdn_b200 import from_spec
     est = from_spec(w["spec"])
@@ -446,6 +461,11 @@ def measure_gpu(w, steps, warmup, world, device, peaks, extras_light=False, cloc
     est.sync_check()
     ms = ev0.elapsed_time(ev1)
     kernel_ms = ms / steps
+    labels = None
+    if keep_labels:   # lab_dev still holds the last timed step's result (batch (steps - 1) % ring)
+        pick = dump_sample(rows)
+        kept = lab_dev if pick is None else lab_dev[torch.from_numpy(pick).to(device)]
+        labels = kept.cpu().numpy().astype(np.float32)
     # keep the very same work running for ~1.5 s so that nvidia-smi (100 ms period) sees the clocks under this load
     load_window = None
     if clock_probe_s > 0:
@@ -570,7 +590,7 @@ def measure_gpu(w, steps, warmup, world, device, peaks, extras_light=False, cloc
                          indices_value=e2e_indices, indices_call="estimator.predict_indices(X, out=page-locked int32): no label materialisation",
                          pageable_value=e2e_pageable, pageable_call="estimator.predict(X) on rows in pageable host memory",
                          bound="PCIe: host rows cross at ~48-55 GB/s per GPU; the streaming models' kernels are 50-100x faster than the copy"),
-                roofline=roofline, est=est, batch0=batches[0])
+                roofline=roofline, est=est, batch0=batches[0], labels=labels)
 
 
 def _threadpools():
@@ -599,6 +619,9 @@ class _SvcPool:
 
     def close(self):
         self.par.__exit__(None, None, None)
+        # joblib keeps loky's workers alive for reuse after the Parallel block: stop them, so none outlives the bench
+        from joblib.externals.loky import get_reusable_executor
+        get_reusable_executor(reuse=True).shutdown(wait=True)
 
 
 def cpu_reference(w, max_seconds=20.0, steps=2, warmup=1):
@@ -757,7 +780,12 @@ def main():
     ap.add_argument("--gpu-only", action="store_true", help="skip the scikit-learn baselines (tuning sweeps)")
     ap.add_argument("--set-option", action="append", default=[], metavar="KEY=VALUE",
                     help="tcsdn_set_option on every estimator (include/tcsdn.h TCSDN_OPT_*), e.g. 4=3")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the label indices each workload's last timed step computed as "
+                         "DIR/<workload>_labels.npy (float32; a fixed, seeded sample of 1Mi rows where a step has more)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     for kv in args.set_option:
         OPTIONS.append((int(kv.split("=")[0]), int(kv.split("=")[1])))
     args.warmup = max(args.warmup, 3)
@@ -796,7 +824,10 @@ def main():
     w = build_workload(args.workload, args.quick)
     sampler = ClockSampler(local)
     sampler.start()
-    head = measure_gpu(w, args.steps, args.warmup, world, device, peaks, clock_probe_s=1.5)
+    dump = bool(args.dump_outputs) and rank == 0
+    outputs = {}
+    head = measure_gpu(w, args.steps, args.warmup, world, device, peaks, clock_probe_s=1.5, keep_labels=dump)
+    outputs[args.workload] = head["labels"]
     clocks = sampler.stop(*head["load_window"])
     clocks["how"] = "nvidia-smi -lms 100 over a 1.5 s continuation of the timed CUDA graph (same kernels, same batches)"
 
@@ -805,8 +836,8 @@ def main():
         for name in [x for x in args.extras.split(",") if x and x != args.workload]:
             try:
                 wx = build_workload(name, args.quick)
-                steps_x = max(3, min(args.steps, 5))
-                r = measure_gpu(wx, steps_x, 3, world, device, peaks, extras_light=True)
+                r = measure_gpu(wx, args.steps, 3, world, device, peaks, extras_light=True, keep_labels=dump)
+                outputs[name] = r["labels"]
                 entry = {"workload": wx["desc"], "dtype": DTYPES.get(wx["spec"]["kind"]), "value": r["value"], "unit": "flow-rows/s", "rows_per_gpu_per_step": r["rows"],
                          "ms_per_step": r["ms_per_step"], "e2e": r["e2e"], "roofline": r["roofline"],
                          "gpu_launches_per_step": r["launches_per_step"], "engine_stats": r["est"].stats().tolist(),
@@ -855,6 +886,11 @@ def main():
             if "value" in gathered:
                 line["value_with_gather"] = gathered["value"]
                 line["gather_efficiency"] = gathered["value"] / head["value"]
+        if dump:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, labels in outputs.items():
+                if labels is not None:
+                    np.save(os.path.join(args.dump_outputs, f"{name}_labels.npy"), labels)
         print(json.dumps(line))
     if world > 1:
         import torch.distributed as dist

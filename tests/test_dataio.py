@@ -1,5 +1,6 @@
-"""Training-data reader/writer (SURVEY row N4): format round trip, mixed delimiters, truncated tail, and -- where the
-reference checkout is present (this container, not the GPU box) -- the notebooks' 7 653-row recipe against the golden rows."""
+"""Training-data reader/writer (SURVEY row N4): format round trip, mixed delimiters, truncated tail, and the notebooks'
+recipe on a verbatim sample of the reference's bundled files against the golden rows."""
+import json
 import os
 
 import numpy as np
@@ -8,7 +9,7 @@ import pytest
 from traffic_classifier_sdn_b200 import dataio, flows
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_DATA = "/root/reference/datasets"
+SAMPLE = os.path.join(HERE, "golden", "datasets")
 
 
 def _table():
@@ -75,10 +76,17 @@ def test_errors(tmp_path):
         dataio.load_training_set([])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference checkout not present (GPU box)")
 def test_notebook_recipe_reproduces_the_golden_rows():
+    """The reference's five bundled files, sampled verbatim (tests/golden/make_datasets_sample.py): read in the notebooks'
+    order, every kept line must parse to the golden row pandas made of it, and ping's truncated last line must go."""
     z = np.load(os.path.join(HERE, "golden", "bundled.npz"))
-    paths = [os.path.join(REF_DATA, f"{k}_training_data.csv") for k in ("ping", "voice", "dns", "telnet", "game")]
-    X, y = dataio.load_training_set(paths)
-    assert X.shape == (7653, 12)
-    assert np.array_equal(X, z["X"]) and np.array_equal(y, z["y"].astype(str))
+    with open(os.path.join(SAMPLE, "sample.json")) as fh:
+        meta = json.load(fh)
+    X, y = dataio.load_training_set([os.path.join(SAMPLE, m["file"]) for m in meta])
+    rows, offset = [], 0
+    for m in meta:
+        rows += [offset + i for i in m["lines"] if i < m["rows"]]
+        offset += m["rows"]
+    assert offset == len(z["X"]) == 7653 and len(rows) < sum(len(m["lines"]) for m in meta)
+    assert X.shape == (len(rows), 12)
+    assert np.array_equal(X, z["X"][rows]) and np.array_equal(y, z["y"][rows].astype(str))
